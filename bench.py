@@ -96,6 +96,19 @@ def emit_result(line: dict):
 
 SEED_SCALARS, SEED_POINTS, SEED_NTT = 0xB2000001, 0xB2000002, 0xB2000003
 R_MOD = 0x30644E72E131A029B85045B68181585D2833E84879B9709143E1F593F0000001
+# --dump-outputs keeps a fixed, seeded sample of DUMP_ELEMS elements of a long vector (a 2^24-element Fr vector is 512 MiB)
+SEED_DUMP, DUMP_ELEMS = 0xB2000004, 1 << 16
+
+
+def dump_outputs(out_dir: str, outputs: dict):
+    """--dump-outputs: out_dir/<name>.npy for every output of the last timed step, so that two builds run with the same
+    arguments can be compared output for output.  Each output is the bytes a caller receives (encoded points, proof
+    bytes, field elements as little-endian limbs), one float32 per byte: exact, so a difference in any bit shows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, raw in outputs.items():
+        a = np.frombuffer(raw, dtype=np.uint8) if isinstance(raw, bytes) else raw
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def source_hash() -> str:
@@ -215,8 +228,10 @@ def run_reference(args):
         cpu_msm_sample(min(log_sample, 16))
     times, rate = [], 0.0
     for _ in range(args.steps):
-        rate, dt, cores, _, _ = cpu_msm_sample(log_sample)
+        rate, dt, cores, out, _ = cpu_msm_sample(log_sample)
         times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"g1_msm": out})
     ms = 1e3 * sum(times) / len(times)
     value = (1 << log_sample) / (ms / 1e3)
     ntt_rate, ntt_dt = cpu_ntt_sample(min(22, args.log_n))
@@ -324,7 +339,7 @@ def run_gpu(args):
         table_setup_s = time.perf_counter() - t0  # one-off per proving key, OUTSIDE every timed region (reported, not hidden)
     elif args.window:
         ctx.set_msm_window(args.window)
-    result = {}
+    result, dumps = {}, {}
 
     from ethrex_b200.dist import msm_sharded, shard_range
 
@@ -368,6 +383,7 @@ def run_gpu(args):
 
     msm_step_stats = {}
     ms_step, launches, clocks = timed_loop(msm_step, args.steps, args.warmup, msm_step_stats)
+    dumps["g1_msm"] = result["out"]
     value = world * n / (ms_step / 1e3)
 
     # ---- correctness of what was timed: closed form of the chain MSM (rank 0, outside the timed region)
@@ -454,7 +470,7 @@ def run_gpu(args):
     if not args.no_plain and world == 1 and not args.no_precompute:
         hp = ctx.g1_bases_from_device(d_points, n)
         st = {}
-        pms, _, _ = timed_loop(lambda: result.__setitem__("plain", ctx.g1_msm_resident_device(hp, d_scalars, n)), max(3, args.steps // 2), 2, st)
+        pms, _, _ = timed_loop(lambda: result.__setitem__("plain", ctx.g1_msm_resident_device(hp, d_scalars, n)), args.steps, 2, st)
         ctx.bases_free(hp)
         assert result["plain"] == result["out"]
         plain = {"value": n / (pms / 1e3), "unit": "points/s", "ms_per_step": pms,
@@ -497,8 +513,9 @@ def run_gpu(args):
         ctx.synchronize()
         g2_setup = time.perf_counter() - t0
         st2 = {}
-        g2_steps = max(3, args.steps // 2)
+        g2_steps = args.steps
         g2ms, g2l, _ = timed_loop(lambda: result.__setitem__("g2", ctx.g2_msm_resident_device(h2, d_scalars, g2n)), g2_steps, 2, st2)
+        dumps["g2_msm"] = result["g2"]
         g2_ok = None
         if not args.no_verify:
             g2_ok = bool(closed_form(g2n, SEED_SCALARS, g2=True) == result["g2"])
@@ -549,7 +566,8 @@ def run_gpu(args):
             ctx.bases_precompute(hs_, 0)
             sc = torch.empty(4 * m, dtype=torch.int64, device="cuda")
             ctx.fr_random_device(sc, m, SEED_SCALARS, lo)
-            sms, _, _ = timed_loop(lambda: result.__setitem__("s" + tag, msm_sharded(ctx, None, sc, m, g2=is_g2, handle=hs_)), max(3, args.steps // 2), 2)
+            sms, _, _ = timed_loop(lambda: result.__setitem__("s" + tag, msm_sharded(ctx, None, sc, m, g2=is_g2, handle=hs_)), args.steps, 2)
+            dumps[f"strong_{tag}_msm"] = result["s" + tag]
             ctx.bases_free(hs_)
             del sc
             torch.cuda.empty_cache()
@@ -571,7 +589,7 @@ def run_gpu(args):
                         result["one" + tag] = fn1(h1, sc1, n)
                     torch.cuda.synchronize()
                     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    reps = 3
+                    reps = args.steps
                     e0.record()
                     for _ in range(reps):
                         fn1(h1, sc1, n)
@@ -597,10 +615,16 @@ def run_gpu(args):
         d_ntt = torch.empty(4 * n, dtype=torch.int64, device="cuda")
         ctx.fr_random_device(d_ntt, n, SEED_NTT, start, eb.SCALARS_MONT)
         ref = d_ntt.clone()
+        rows = torch.from_numpy(np.sort(np.random.default_rng(SEED_DUMP).choice(n, min(n, DUMP_ELEMS), replace=False)))
+
+        def sample(t):
+            return t.view(n, 4)[rows.to(t.device)].cpu().numpy().view(np.uint8)
         fwd_ms, fl, _ = timed_loop(lambda: ctx.fr_ntt_device(d_ntt, log_n, 0), args.steps, args.warmup)
+        dumps["ntt_forward"] = sample(d_ntt)
         d_ntt.copy_(ref)
         ctx.fr_ntt_device(d_ntt, log_n, 0)
         inv_ms, _, _ = timed_loop(lambda: ctx.fr_ntt_device(d_ntt, log_n, eb.NTT_INVERSE), args.steps, args.warmup)
+        dumps["ntt_inverse"] = sample(d_ntt)
         # round trip check on fresh data
         d_ntt.copy_(ref)
         ctx.fr_ntt_device(d_ntt, log_n, 0)
@@ -623,7 +647,8 @@ def run_gpu(args):
         if not args.no_e2e and world == 1:
             h_ntt = torch.empty(4 * n, dtype=torch.int64).pin_memory()
             h_ntt.copy_(ref)
-            wall = wall_loop(lambda: ctx.fr_ntt(h_ntt, log_n, 0), max(2, args.steps // 2), 1)
+            wall = wall_loop(lambda: ctx.fr_ntt(h_ntt, log_n, 0), args.steps, 1)
+            dumps["ntt_forward_e2e"] = sample(h_ntt)
             ntt["e2e"] = {"value": n / wall, "unit": "elements/s", "ms_per_step": wall * 1e3, "h2d_bytes_per_step": 32 * n, "d2h_bytes_per_step": 32 * n,
                           "api": "b200zk_fr_ntt (pinned host buffer, in place): PCIe-bound, 2 x 512 MiB per transform"}
             del h_ntt
@@ -643,12 +668,13 @@ def run_gpu(args):
         backend = B200Backend(ctx, circuit)
         backend.prove({"batch": 0})  # warm-up (workspaces, twiddles)
         times, digests, pl0 = [], [], ctx.launch_count
-        reps = max(2, min(args.steps, 5))
+        reps = args.steps
         for i in range(reps):
             barrier()
             pr, dt = backend.prove_timed({"batch": i + 1}, ProofFormat.GROTH16)
             times.append(max_over_ranks(dt))
             digests.append(pr.proof.hex()[:16])
+        dumps["groth16_proof"] = pr.proof
         proof_launches = (ctx.launch_count - pl0) // reps
         # same bytes on every rank (the fold is replicated)
         if world > 1:
@@ -716,6 +742,8 @@ def run_gpu(args):
             "g2": g2, "strong": strong, "ntt": ntt, "proof": proof, "cpu_baseline": cpu,
         }
         emit_result(line)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumps)
     ctx.close()
     if world > 1:
         dist.destroy_process_group()
@@ -744,7 +772,10 @@ def main():
     ap.add_argument("--no-proof-separate", action="store_true")
     ap.add_argument("--no-precompute", action="store_true", help="plain resident bases (no 2^(cw) P_i table)")
     ap.add_argument("--window", type=int, default=0, help="force the MSM window bits (0 = automatic)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of each timed path computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
